@@ -28,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree: it leaves nothing in it
 
 METRIC = "tokens/sec (device-timed) Llama-7B-shape ONNX decode, 1/2/4/8 B200 + CPU ref"
 POS = 511
@@ -47,7 +48,24 @@ def parse():
                          "an extra line beside the bf16 headline, never the headline itself")
     ap.add_argument("--config", default="llama", choices=["llama", "gpt2", "resnet50"],
                     help="llama (default) = BASELINE configs[2] / [4], the headline; gpt2 = configs[1]; resnet50 = configs[3] (single GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32): llama: logits "
+                         "[batch, 1, vocab] and the K / V cache rows the step appended [layers, batch, heads, head_dim] (rank 0's "
+                         "heads under tensor parallelism); gpt2 / resnet50: the graph output. Inputs are seeded: two builds run "
+                         "with the same arguments can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    return a
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 # ------------------------------------------------------------------------------------------ CPU arm
@@ -344,6 +362,15 @@ def run_b200(args):
     e2e_ms = max_over_ranks(max(e0.elapsed_time(e1), wall_ms)) / args.steps
     clocks = sampler.stop() if sampler else None
     logits_finite = bool(torch.isfinite(logits_host.float()).all())
+    if args.dump_outputs and rank == 0:
+        rows = {"k_cache_rows": [], "v_cache_rows": []}
+        for name, caches in (("k_cache_rows", g.k_caches), ("v_cache_rows", g.v_caches)):
+            for t in caches:  # [batch, heads, s_max, head_dim]: the row at POS is what the step appended
+                full = torch.empty(t.shape(), dtype=torch.bfloat16, device="cuda")
+                L.check(L.lib.it_b200_copy(ctypes.c_void_p(t.device_ptr()), ctypes.c_void_p(full.data_ptr()), t.nbytes(), ts))
+                rows[name].append(full[:, :, POS].float())
+        dump_outputs(args.dump_outputs, {"logits": logits_host.float().numpy(),
+                                         **{name: torch.stack(r).cpu().numpy() for name, r in rows.items()}})
 
     # ---- roofline of the dominant kernel (gemm_skinny_kernel): all MatMuls of one step, back to back on the
     # runtime stream, CUDA events around them, repeated; algorithmic bytes = weight + activation in/out bytes
@@ -585,6 +612,8 @@ def run_model_config(args):
     e1.synchronize()
     e2e_ms = max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3) / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"output": out_host.float().numpy()})
     pk = {}
     try:
         pk = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

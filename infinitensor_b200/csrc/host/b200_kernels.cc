@@ -7,7 +7,7 @@
 // SEAM-A BUILD (-DITB_SEAM_A, oracle/Makefile target `seam_a`): this very file is compiled against the REFERENCE's own headers
 // (/root/reference/include: core/kernel.h:32-195, cuda/cuda_kernel_wihtout_config.h, cuda/cuda_runtime.h, operators/*.h) and
 // linked, together with libit_b200.so, in place of the reference's src/kernels/cuda directory; the reference's gtests then
-// run against these kernels (tests/test_gpu_seam_a.py).  Only what does not exist in the reference is compiled out there:
+// run against these kernels (oracle/_ref/seam_a/seam_a_tests).  Only what does not exist in the reference is compiled out there:
 // the fused executors of this repo's schedule, the per-row-position extension and the dlopen'ed NCCL collectives.
 #ifdef ITB_SEAM_A
 #include "core/kernel.h"
